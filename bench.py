@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- rays/sec of the NeRF ray-marching hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--mode forward|train] [--impl b200|reference|torch_gpu]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--mode forward|train] [--impl b200|reference|torch_gpu] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one 4096-ray batch of synthetic lego-shaped rays (BASELINE configs[1]:
 64 coarse + 128 fine samples, 8x256 MLP + 128-wide view head).
@@ -17,6 +17,11 @@ One "step" = one pass of the hot path over one 4096-ray batch of synthetic lego-
   * `cpu_baseline` / `--impl reference`: the reference on the host cores (the unmodified script when baseline/_ref is
     present -- kind "reference" --, else the op-chain port oracle/torch_ref.py -- kind "port").
 JSON keys: see the build spec (value, e2e, roofline, cpu_baseline, clocks, gpu_launches ...).
+--dump-outputs DIR writes what the last timed step of the headline path computed on rank 0 as DIR/<name>.npy (float32), so
+that two builds can be compared output for output (the inputs are seeded: the same arguments give the same inputs).  Forward:
+render()'s rgb_map, disp_map, acc_map and extras (rgb0, disp0, acc0, z_std), deterministic.  --mode train: the step's loss
+(train_loss), the parameters after it (train_params) and its gradient (train_grads), flat in the networks' parameter order;
+the backward accumulates with atomics, so these differ from run to run by rounding that the optimizer steps amplify.
 """
 import argparse
 import ctypes as C
@@ -311,14 +316,17 @@ class ClockSampler:
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=30)
+    ap.add_argument("--steps", type=int, default=30, help="timed steps of each headline measurement")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference", "torch_gpu"])
     ap.add_argument("--mode", default="forward", choices=["forward", "train"], help="which measurement is the headline `value`")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-torch-gpu", action="store_true")
     ap.add_argument("--no-train", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
@@ -370,8 +378,11 @@ def main():
     rays_dev = rays_host.to(dev)
     flush = torch.empty(512 << 20, dtype=torch.uint8, device=dev)            # > 126 MB L2
 
+    last = {}
+
     def timed(fn, steps, warmup, use_events=True):
-        """-> (median ms per step, max over ranks).  L2 flushed between timed iterations, outside the timed region."""
+        """-> (median ms per step, max over ranks); last["out"] is what the last timed call returned.  L2 flushed between
+        timed iterations, outside the timed region."""
         for _ in range(warmup):
             flush.zero_(); fn()
         torch.cuda.synchronize()
@@ -383,11 +394,12 @@ def main():
             flush.zero_()
             if use_events:
                 a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                a.record(); fn(); b.record()
+                a.record(); out = fn(); b.record()
                 evs.append((a, b))
             else:
                 torch.cuda.synchronize()
-                t0 = time.perf_counter(); fn(); walls.append((time.perf_counter() - t0) * 1e3)
+                t0 = time.perf_counter(); out = fn(); walls.append((time.perf_counter() - t0) * 1e3)
+        last["out"] = out
         torch.cuda.synchronize()
         if world > 1:
             dist.barrier()
@@ -426,6 +438,10 @@ def main():
     total_steps = args.warmup + args.steps
     lib.nerf_b200_timing_enable(1)
     ms_res, ms_res_mean = timed(step_resident, args.steps, args.warmup)
+    dump_fwd, dump_train = {}, {}
+    if args.dump_outputs:
+        rgb, disp, acc, extras = last["out"]
+        dump_fwd = {k: v.cpu().numpy() for k, v in dict(rgb_map=rgb, disp_map=disp, acc_map=acc, **extras).items()}
     kms, kn, kfl, _ = read_timing()                 # accumulators hold warm-up + timed launches: per-launch averages are reported
     lib.nerf_b200_timing_enable(0)
     ms_e2e, _ = timed(lambda: graphed(rays_host), args.steps, args.warmup, use_events=False)
@@ -470,6 +486,8 @@ def main():
             lib.nerf_b200_timing_enable(0)
             ms_dev, ms_dev_mean = timed(tr.step_device, args.steps, args.warmup)
             ms_host, _ = timed(lambda: tr(r_h, t_h), args.steps, args.warmup, use_events=False)
+            if args.dump_outputs and not group_world:
+                dump_train.update(train_loss=tr.state[0:1].cpu().numpy(), train_params=tr.flat_p.cpu().numpy(), train_grads=tr.flat_g.cpu().numpy())
             # kernel split of the step: an eager (un-graphed) pass with the library's event bracketing on
             lib.nerf_b200_timing_enable(1)
             for _ in range(3):
@@ -599,6 +617,10 @@ def main():
             ref = _sub_json(["--impl", "reference", "--steps", "3", "--warmup", "1"], env={"CUDA_VISIBLE_DEVICES": ""}, timeout=400)
             line["cpu_baseline"] = ref.get("cpu_baseline", ref)
     if rank == 0:
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for k, v in (dump_fwd if headline is not None else dump_train).items():
+                np.save(os.path.join(args.dump_outputs, k + ".npy"), v.astype(np.float32))
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -1,14 +1,15 @@
-"""Import the UNMODIFIED reference (/root/reference) on CPU  --  build-container only.
+"""Import the UNMODIFIED reference on CPU, for the golden-fixture generators only.
 
+The reference is read from $NERF_REFERENCE, else from the git-ignored copy oracle/_ref/ (oracle/fetch_reference.py).
 imageio / matplotlib are not installed and only used by I/O code paths, so empty module stubs
-are registered first (SURVEY.md 8c).  Nothing on the GPU box may call this (no /root/reference
-there); it exists to pin the oracle and to generate tests/golden/.
+are registered first (SURVEY.md 8c).  No test, smoke() or bench.py calls this; it exists to pin
+the oracle and to generate tests/golden/.
 """
 import os
 import sys
 import types
 
-REF = os.environ.get("NERF_REFERENCE", "/root/reference")
+REF = os.environ.get("NERF_REFERENCE", os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
 
 
 def available():

@@ -1,19 +1,17 @@
-"""The drop-in, EXECUTED: the unmodified reference script (baseline/_ref/run_nerf.py, copied there by tools/fetch_reference.py)
-is imported twice, once as it is and once with `nerf_pytorch_b200.dropin.patch` applied, and its own `train()` runs on
-a small synthetic blender-format dataset written to a temp directory -- argument parsing, data loading, ray batching,
+"""The drop-in against the reference's own training run: the unmodified reference script's `train()` ran K iterations on a
+small synthetic blender-format dataset (oracle/gen_reference_runs.py: argument parsing, data loading, ray batching,
 `create_nerf` (run_nerf.py:640), `render(..., retraw=True)` (:760), the two MSE terms, `loss.backward()`,
-`optimizer.step()` and the learning-rate decay (:764-784) are all the reference's code.  Only three things are
-provided from outside, none of them on the path: an `imageio` stand-in backed by cv2 and a `configargparse` stand-in
-backed by argparse (both packages are absent from this image), and `trange` rebound to stop after a few iterations
-(N_iters = 200001 is hard-coded at run_nerf.py:701).
+`optimizer.step()` and the learning-rate decay (:764-784)), and tests/golden/dropin_train.npz holds what it saw and did:
+each iteration's ray batch, target and CUDA generator state before `render()`, every loss term and a seeded sample of
+the parameter update.  Here the names `nerf_pytorch_b200.dropin.patch` rebinds on a module run the same iterations from
+the same starting weights with the same arguments.
 
-Checks: same loss trajectory, same parameter update after K steps (within the tensor-core budget), same rendered
-image from the same weights through `render(c2w=...)` under no_grad.  Measured values go to gpurun_out/parity_dropin.json."""
+Checks: same loss trajectory, same parameter update after K steps (within the tensor-core budget), same gradients of one
+more step from identical weights and rays, same rendered image from the same weights through `render(c2w=...)` under
+no_grad.  The measured values are also written to parity_dropin.json, next to the other parity records."""
 import argparse
-import importlib.util
 import json
 import os
-import sys
 import types
 
 import numpy as np
@@ -23,186 +21,95 @@ import torch
 from conftest import ROOT, rel_l2
 
 pytestmark = pytest.mark.gpu
-REF = os.path.join(ROOT, "baseline", "_ref")
-K_ITERS = 6
+NET_KEYS = ("network_fn", "network_fine")
 
 
-def _write_dataset(base, n=(8, 2, 2), H=40):
-    import cv2
-    sys.path.insert(0, REF)
-    ang = 0.6911112070083618
-    rng = np.random.default_rng(0)
-    yy, xx = np.mgrid[0:H, 0:H].astype(np.float32) / H
-    k = 0
-    for split, cnt in zip(("train", "val", "test"), n):
-        os.makedirs(os.path.join(base, split), exist_ok=True)
-        frames = []
-        for i in range(cnt):
-            th, ph = 360.0 * k / sum(n), -30.0 + 10.0 * (k % 3)
-            c, s = np.cos(np.radians(th)), np.sin(np.radians(th))
-            cp, sp = np.cos(np.radians(ph)), np.sin(np.radians(ph))
-            t = np.array([[1, 0, 0, 0], [0, 1, 0, 0], [0, 0, 1, 4.0], [0, 0, 0, 1]], np.float64)
-            rp = np.array([[1, 0, 0, 0], [0, cp, -sp, 0], [0, sp, cp, 0], [0, 0, 0, 1]], np.float64)
-            rt = np.array([[c, 0, -s, 0], [0, 1, 0, 0], [s, 0, c, 0], [0, 0, 0, 1]], np.float64)
-            c2w = np.array([[-1, 0, 0, 0], [0, 0, 1, 0], [0, 1, 0, 0], [0, 0, 0, 1]], np.float64) @ rt @ rp @ t
-            disc = ((xx - 0.5) ** 2 + (yy - 0.5) ** 2) < 0.12
-            img = np.zeros((H, H, 4), np.float32)
-            img[..., 0] = 0.5 + 0.5 * np.sin(6 * xx + th / 40.0)
-            img[..., 1] = 0.5 + 0.5 * np.cos(5 * yy + 0.3 * k)
-            img[..., 2] = 0.3 + 0.4 * xx * yy + 0.2 * rng.random()
-            img[..., 3] = disc
-            img[..., :3] *= disc[..., None]
-            png = (np.clip(img[..., [2, 1, 0, 3]], 0, 1) * 255).astype(np.uint8)          # cv2 writes BGRA
-            cv2.imwrite(os.path.join(base, split, f"r_{i}.png"), png)
-            frames.append({"file_path": f"./{split}/r_{i}", "transform_matrix": c2w.tolist()})
-            k += 1
-        with open(os.path.join(base, f"transforms_{split}.json"), "w") as f:
-            json.dump({"camera_angle_x": ang, "frames": frames}, f)
+def _sampled(fx, kind, tensors):
+    """{name: (ours at the stored indices, reference's stored values)} for every parameter tensor"""
+    out = {}
+    for key in NET_KEYS:
+        for k, t in tensors(key):
+            idx = fx[f"{kind}.{key}.{k}.idx"]
+            out[f"{key}.{k}"] = (t.detach().double().reshape(-1).cpu().numpy()[idx], fx[f"{kind}.{key}.{k}.val"])
+    return out
 
 
-def _stand_ins():
-    import cv2
-    imageio = types.ModuleType("imageio")
-    imageio.imread = lambda f, *a, **k: cv2.imread(f, cv2.IMREAD_UNCHANGED)[..., [2, 1, 0, 3]]
-    imageio.imwrite = lambda f, im, *a, **k: cv2.imwrite(f, np.asarray(im)[..., ::-1])
-    imageio.mimwrite = lambda *a, **k: None
-    cfg = types.ModuleType("configargparse")
-
-    class ArgumentParser(argparse.ArgumentParser):
-        def add_argument(self, *a, **k):
-            k.pop("is_config_file", None)
-            return super().add_argument(*a, **k)
-    cfg.ArgumentParser = ArgumentParser
-    mpl, plt = types.ModuleType("matplotlib"), types.ModuleType("matplotlib.pyplot")
-    mpl.pyplot = plt
-    for name, mod in (("imageio", imageio), ("configargparse", cfg), ("matplotlib", mpl), ("matplotlib.pyplot", plt)):
-        sys.modules.setdefault(name, mod)
-
-
-def _import_reference(alias):
-    spec = importlib.util.spec_from_file_location(alias, os.path.join(REF, "run_nerf.py"))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
-
-
-def _run_train(mod, argv, init_from=None):
-    """run the module's own train() for K_ITERS iterations; returns (create_nerf outputs, initial weights, losses)"""
-    captured, losses = {}, []
-    orig_create = mod.create_nerf
-
-    def spy_create(args):
-        out = orig_create(args)
-        nets = [out[0]["network_fn"], out[0]["network_fine"]]
-        if init_from is not None:
-            for n, sd in zip(nets, init_from):
-                n.load_state_dict(sd)
-        captured["out"] = out
-        captured["init"] = [{k: v.detach().clone() for k, v in n.state_dict().items()} for n in nets]
-        return out
-    orig_mse = mod.img2mse
-
-    def spy_mse(x, y):
-        v = orig_mse(x, y)
-        losses.append(v.detach())
-        return v
-    mod.create_nerf, mod.img2mse = spy_create, spy_mse
-    mod.trange = lambda a, b: range(a, a + K_ITERS)
-    old_argv = sys.argv
-    sys.argv = ["run_nerf.py"] + argv
-    np.random.seed(0)
-    torch.manual_seed(0)
-    try:
-        mod.train()
-    finally:
-        sys.argv = old_argv
-    torch.cuda.synchronize()
-    return captured["out"], captured["init"], [float(v) for v in losses]
-
-
-@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "run_nerf.py")), reason="baseline/_ref missing (run tools/fetch_reference.py where /root/reference exists)")
-def test_reference_train_runs_unchanged_through_the_dropin(tmp_path):
+def test_reference_train_runs_unchanged_through_the_dropin(tmp_path, golden):
     import nerf_pytorch_b200 as nb
     from nerf_pytorch_b200 import dropin
-    _stand_ins()
-    sys.path.insert(0, REF)
-    data = str(tmp_path / "data")
-    _write_dataset(data)
-    argv = ["--datadir", data, "--dataset_type", "blender", "--basedir", str(tmp_path / "logs"), "--N_rand", "512",
-            "--N_samples", "64", "--N_importance", "128", "--use_viewdirs", "--white_bkgd", "--lrate_decay", "500", "--raw_noise_std", "0"]
+    from oracle import synth
+    fx = golden("dropin_train")
+    K_ITERS = fx["rays"].shape[0]
+    args = argparse.Namespace(**json.loads(str(fx["args"])), basedir=str(tmp_path), expname="patched")
+    os.makedirs(tmp_path / "patched")
+    init = [synth.nerf_state(0), synth.nerf_state(1)]
     torch.set_default_tensor_type("torch.cuda.FloatTensor")            # what run_nerf.py:876 does under __main__
     try:
         launches0 = nb.launch_count()
-        ref = _import_reference("run_nerf_reference")
-        out_r, init_r, loss_r = _run_train(ref, argv + ["--expname", "ref"])
-        assert nb.launch_count() == launches0                          # the unpatched run never touched the library
-        pat = dropin.patch(_import_reference("run_nerf_patched"), set_default_device=False)
-        out_p, init_p, loss_p = _run_train(pat, argv + ["--expname", "patched"], init_from=init_r)
+        pat = dropin.patch(types.ModuleType("run_nerf"), set_default_device=False)
+        tr, te, start, grad_vars, optimizer = pat.create_nerf(args)
+        assert isinstance(tr["network_fn"], nb.NeRF) and start == 0
+        for key, sd in zip(NET_KEYS, init):
+            tr[key].load_state_dict({k: torch.from_numpy(v) for k, v in sd.items()})
+        for kw in (tr, te):
+            kw.update(near=2., far=6.)                                  # blender bounds (run_nerf.py:573-574)
+        H = W = 40
+        focal = 0.5 * W / np.tan(0.5 * 0.6911112070083618)
+        K = np.array([[focal, 0, 0.5 * W], [0, focal, 0.5 * H], [0, 0, 1]])
+        # the reference's loop body (run_nerf.py:760-784) on the batches its train() drew, from its generator states
+        losses = []
+        for i in range(K_ITERS):
+            torch.cuda.set_rng_state(torch.from_numpy(fx["rng_state"][i]))
+            target = torch.from_numpy(fx["target"][i]).cuda()
+            rgb, disp, acc, extras = pat.render(H, W, K, chunk=args.chunk, rays=torch.from_numpy(fx["rays"][i]).cuda(), verbose=i < 10,
+                                                retraw=True, **tr)
+            optimizer.zero_grad()
+            terms = [nb.img2mse(rgb, target), nb.img2mse(extras["rgb0"], target)]
+            losses += [float(t) for t in terms]
+            (terms[0] + terms[1]).backward()
+            optimizer.step()
+            for g in optimizer.param_groups:                            # global_step = start + i (run_nerf.py:779-783, :873)
+                g["lr"] = args.lrate * 0.1 ** ((start + i) / (args.lrate_decay * 1000))
+        torch.cuda.synchronize()
         assert nb.launch_count() > launches0
-        assert isinstance(out_p[0]["network_fn"], nb.NeRF) and not isinstance(out_r[0]["network_fn"], nb.NeRF)
-        stats = {"loss_reference": loss_r, "loss_patched": loss_p}
-        assert len(loss_r) == len(loss_p) == 2 * K_ITERS                # img2mse is called twice per iteration (:764, :771)
-        stats["loss_max_rel_dev"] = float(np.max(np.abs(np.array(loss_p) - np.array(loss_r)) / np.array(loss_r)))
-        # parameter update after K iterations (Adam, same lr schedule): patched vs unpatched
+        loss_r = fx["loss"]
+        assert len(losses) == len(loss_r) == 2 * K_ITERS                # img2mse is called twice per iteration (:764, :771)
+        stats = {"loss_reference": loss_r.tolist(), "loss_patched": losses}
+        stats["loss_max_rel_dev"] = float(np.max(np.abs(np.array(losses) - loss_r) / loss_r))
+        # parameter update after K iterations (Adam, same lr schedule), on the stored sample of every tensor
         upd = {}
-        for tag, i in (("coarse", 0), ("fine", 1)):
-            key = "network_fn" if i == 0 else "network_fine"
-            sd_r, sd_p = out_r[0][key].state_dict(), out_p[0][key].state_dict()
-            for k in sd_r:
-                dr = (sd_r[k] - init_r[i][k]).double().reshape(-1).cpu().numpy()
-                dp = (sd_p[k] - init_r[i][k]).double().reshape(-1).cpu().numpy()
-                upd[f"{tag}.{k}"] = {"rel": rel_l2(dp, dr), "cos": float(dp @ dr / (np.linalg.norm(dp) * np.linalg.norm(dr) + 1e-30))}
+        init_t = {key: {k: torch.from_numpy(v).cuda() for k, v in sd.items()} for key, sd in zip(NET_KEYS, init)}
+        for name, (dp, dr) in _sampled(fx, "upd", lambda key: [(k, v - init_t[key][k]) for k, v in tr[key].state_dict().items()]).items():
+            upd[name] = {"rel": rel_l2(dp, dr), "cos": float(dp @ dr / (np.linalg.norm(dp) * np.linalg.norm(dr) + 1e-30))}
         stats["update"] = upd
         stats["update_cos_min"] = min(v["cos"] for v in upd.values())
         stats["update_rel_median"] = float(np.median([v["rel"] for v in upd.values()]))
-        # gradients of one more reference-style step from IDENTICAL weights and rays (perturb = 0), patched vs unpatched:
+        # gradients of one more reference-style step from IDENTICAL weights and rays (perturb = 0):
         # Adam's first steps move every element by ~lr * sign(g), so elements whose gradient is noise-level make the
         # UPDATE vectors of some tensors decorrelate (recorded above) even when the gradients agree; the gate is on the gradients
-        for key in ("network_fn", "network_fine"):
-            out_p[0][key].load_state_dict(out_r[0][key].state_dict())
-        H0 = W0 = 40
-        f0 = 0.5 * W0 / np.tan(0.5 * 0.6911112070083618)
-        K0 = np.array([[f0, 0, 0.5 * W0], [0, f0, 0.5 * H0], [0, 0, 1]])
-        pose = torch.Tensor(np.array(json.load(open(os.path.join(data, "transforms_train.json")))["frames"][1]["transform_matrix"])[:3, :4])
-        ro, rd = ref.get_rays(H0, W0, K0, pose)
-        sel = torch.randperm(H0 * W0)[:512]
-        batch_rays = torch.stack([ro.reshape(-1, 3)[sel], rd.reshape(-1, 3)[sel]], 0)
-        tgt = torch.rand(512, 3)
-        gstats = {}
-        grads = {}
-        for tag, mod, out in (("ref", ref, out_r), ("pat", pat, out_p)):
-            kw = dict(out[0]); kw.update(near=2., far=6., perturb=0.)
-            for key in ("network_fn", "network_fine"):
-                for p_ in kw[key].parameters():
-                    p_.grad = None
-            rgb, disp, acc, extras = mod.render(H0, W0, K0, chunk=32768, rays=batch_rays, verbose=False, retraw=True, **kw)
-            loss = mod.img2mse(rgb, tgt) + mod.img2mse(extras["rgb0"], tgt)
-            loss.backward()
-            grads[tag] = {f"{key}.{k}": p_.grad.detach().double().reshape(-1).cpu().numpy()
-                          for key in ("network_fn", "network_fine") for k, p_ in kw[key].named_parameters()}
-        for k in grads["ref"]:
-            gstats[k] = rel_l2(grads["pat"][k], grads["ref"][k])
+        for key, sd in zip(NET_KEYS, init):
+            tr[key].load_state_dict({k: torch.from_numpy(v) for k, v in sd.items()})
+        kw = dict(tr); kw.update(perturb=0.)
+        for key in NET_KEYS:
+            for p_ in kw[key].parameters():
+                p_.grad = None
+        tgt = torch.from_numpy(fx["grad_target"]).cuda()
+        rgb, disp, acc, extras = pat.render(H, W, K, chunk=32768, rays=torch.from_numpy(fx["grad_rays"]).cuda(), verbose=False, retraw=True, **kw)
+        (nb.img2mse(rgb, tgt) + nb.img2mse(extras["rgb0"], tgt)).backward()
+        grads = _sampled(fx, "grad", lambda key: [(k, p_.grad) for k, p_ in kw[key].named_parameters()])
+        gstats = {name: rel_l2(gp, gr) for name, (gp, gr) in grads.items()}
         stats["grad_rel"] = gstats
         stats["grad_rel_median"] = float(np.median(list(gstats.values())))
         stats["grad_rel_max"] = float(max(gstats.values()))
-        allr, allp = np.concatenate(list(grads["ref"].values())), np.concatenate(list(grads["pat"].values()))
+        allp = np.concatenate([gp for gp, _ in grads.values()])
+        allr = np.concatenate([gr for _, gr in grads.values()])
         stats["grad_cos_all"] = float(allr @ allp / (np.linalg.norm(allr) * np.linalg.norm(allp)))
         # same weights -> same image through render(c2w=...) under no_grad (run_nerf.py:154 call shape)
-        for key in ("network_fn", "network_fine"):
-            out_p[1][key].load_state_dict(out_r[1][key].state_dict())
-        H = W = 40
-        focal = 0.5 * W / np.tan(0.5 * 0.6911112070083618)
-        Km = np.array([[focal, 0, 0.5 * W], [0, focal, 0.5 * H], [0, 0, 1]])
-        c2w = torch.Tensor(np.array(json.load(open(os.path.join(data, "transforms_test.json")))["frames"][0]["transform_matrix"])[:3, :4])
-        kw_r, kw_p = dict(out_r[1]), dict(out_p[1])
-        for kw in (kw_r, kw_p):
-            kw.update(near=2., far=6.)
         with torch.no_grad():
-            img_r = ref.render(H, W, Km, chunk=32768, c2w=c2w, **kw_r)
-            img_p = pat.render(H, W, Km, chunk=32768, c2w=c2w, **kw_p)
-        stats["render_rgb_rel"] = rel_l2(img_p[0].cpu().numpy(), img_r[0].cpu().numpy())
-        stats["render_acc_rel"] = rel_l2(img_p[2].cpu().numpy(), img_r[2].cpu().numpy())
-        stats["render_rgb0_rel"] = rel_l2(img_p[3]["rgb0"].cpu().numpy(), img_r[3]["rgb0"].cpu().numpy())
+            img_p = pat.render(H, W, K, chunk=32768, c2w=torch.from_numpy(fx["c2w"]).cuda(), **te)
+        stats["render_rgb_rel"] = rel_l2(img_p[0].cpu().numpy(), fx["render_rgb"])
+        stats["render_acc_rel"] = rel_l2(img_p[2].cpu().numpy(), fx["render_acc"])
+        stats["render_rgb0_rel"] = rel_l2(img_p[3]["rgb0"].cpu().numpy(), fx["render_rgb0"])
         os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
         with open(os.path.join(ROOT, "gpurun_out", "parity_dropin.json"), "w") as f:
             json.dump(stats, f, indent=1)

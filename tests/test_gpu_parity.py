@@ -180,18 +180,14 @@ def test_psnr_on_the_analytic_scene_matches_the_reference(G):
 def test_reference_tf32_deviates_as_much(G):
     """Context for the tensor-core gates: the UNMODIFIED reference on this GPU with TF32 matmuls (the default of its pinned torch
     1.11; same 10-bit mantissa as our fp16 operands) against its own fp32 run on the same GPU, next to our tc_fp16 path against
-    that fp32 run -- on the trained networks, 1024 lego rays."""
-    import ref_gpu
-    if not ref_gpu.available():
-        pytest.skip("baseline/_ref missing")
+    that fp32 run -- on the trained networks, 1024 lego rays.  The reference's two GPU runs are stored in
+    tests/golden/reference_gpu_trained_lego_1024.npz (oracle/gen_reference_runs.py)."""
     fx = load_golden("trained_lego_1024")
     sb = G.synth.ray_batch("lego", int(fx["N"]), seed=int(fx["ray_seed"]))
-    w = load_golden("trained_weights")
-    sc = {k[2:]: v for k, v in w.items() if k.startswith("c.")}
-    sf = {k[2:]: v for k, v in w.items() if k.startswith("f.")}
-    mod = ref_gpu.load()
-    r32 = ref_gpu.render(mod, sc, sf, sb["H"], sb["W"], sb["K"], sb["rays"], tf32=False)
-    rtf = ref_gpu.render(mod, sc, sf, sb["H"], sb["W"], sb["K"], sb["rays"], tf32=True)
+    rg = load_golden("reference_gpu_trained_lego_1024")
+    assert int(rg["N"]) == int(fx["N"]) and int(rg["ray_seed"]) == int(fx["ray_seed"])
+    r32 = {k: rg["fp32_" + k] for k in ("rgb_map", "acc_map", "rgb0", "acc0")}
+    rtf = {k: rg["tf32_" + k] for k in ("rgb_map", "acc_map", "rgb0", "acc0")}
     nets = _trained_nets(G)
     with torch.no_grad():
         rgb, disp, acc, ex = G.nb.render(sb["H"], sb["W"], sb["K"], chunk=32768, rays=G.dev(sb["rays"]), ndc=False, near=2., far=6., use_viewdirs=True,

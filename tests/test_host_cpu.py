@@ -137,32 +137,29 @@ def test_cached_parameter_list_follows_the_module(nb):
     assert [k for _, _, k, _ in plain._named_params()] == [k for k, _ in plain.named_parameters()]
 
 
-def test_keras_weight_import_matches_the_reference(nb):
+def test_keras_weight_import_matches_the_reference(nb, golden):
     """NeRF.load_weights_from_keras vs the reference's own (run_nerf_helpers.py:121-148) on a synthetic Keras-style weight list;
-    needs /root/reference (build container), otherwise checks the documented layout only."""
-    rng = np.random.default_rng(0)
-    shapes = [(63, 256)] + [(256, 256)] * 4 + [(319, 256)] + [(256, 256)] * 2 + [(256, 256), (283, 128), (128, 3), (256, 1)]
-    weights = []
-    for (i, o) in shapes:
-        weights += [rng.standard_normal((i, o)).astype(np.float32), rng.standard_normal((o,)).astype(np.float32)]
+    the reference's state_dict (keys in order, shapes, a seeded sample of the entries) is tests/golden/keras_weights.npz."""
+    from oracle.gen_reference_runs import keras_weight_list
+    weights = keras_weight_list()
     m = nb.NeRF(D=8, W=256, input_ch=63, input_ch_views=27, output_ch=5, skips=[4], use_viewdirs=True)
     m.load_weights_from_keras(weights)
     assert torch.equal(m.pts_linears[5].weight, torch.from_numpy(weights[10].T)) and torch.equal(m.alpha_linear.bias, torch.from_numpy(weights[23]))
-    from oracle import ref_import
-    if ref_import.available():
-        _, rh = ref_import.load()
-        r = rh.NeRF(D=8, W=256, input_ch=63, input_ch_views=27, output_ch=5, skips=[4], use_viewdirs=True)
-        r.load_weights_from_keras(weights)
-        for (ka, a), (kb, b) in zip(m.state_dict().items(), r.state_dict().items()):
-            assert ka == kb and torch.equal(a, b), ka
+    ref = golden("keras_weights")
+    sd = m.state_dict()
+    assert list(sd.keys()) == [str(k) for k in ref["keys"]]
+    for k, a in sd.items():
+        assert list(a.shape) == ref[f"{k}__shape"].tolist(), k
+        assert np.array_equal(a.numpy().reshape(-1)[ref[f"{k}__idx"]], ref[f"{k}__val"]), k
 
 
-def test_dropin_patch_list_covers_the_seam(nb):
+def test_dropin_patch_list_covers_the_seam(nb, monkeypatch):
     from nerf_pytorch_b200 import dropin
     for name in ("render", "render_rays", "batchify_rays", "raw2outputs", "create_nerf", "sample_pdf", "NeRF", "get_embedder"):
         assert name in dropin.PATCHED and hasattr(nb, name)
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)      # also where a GPU is present
     with pytest.raises(RuntimeError):
-        dropin.patch(types.ModuleType("run_nerf"))        # no CUDA here -> refuses
+        dropin.patch(types.ModuleType("run_nerf"))        # no CUDA -> refuses
 
 
 def test_bench_reference_arm_runs_on_cpu():
