@@ -270,10 +270,6 @@ int nerf_b200_mse_seed(const float* rgb, const float* target, int64_t N, float g
 int nerf_b200_adam_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n, float* state,
                         float lr0, float decay_rate, float decay_steps, float beta1, float beta2, float eps, float grad_mul, void* stream);
 
-/* ---- debug hook (NERF_B200_TRACE builds only; a no-op otherwise): clock64 trace of CTA 0 into a device
- *      buffer of 4096 int64 (NULL disables) ---------------------------------------------------------------- */
-int nerf_b200_debug_set_trace(void* dev_buf_4096_i64);
-
 /* ---- device-time accounting of the dominant kernels (march_tc2 / dgrad_tc2 / wgrad_tc) for bench.py's roofline:
  *      when enabled, every launch is bracketed by CUDA events on its own stream; read() synchronises
  *      those events, returns the summed kernel time [ms], the launch count and the algorithmic

@@ -8,9 +8,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# NERF_B200_EXPERIMENTS=1 selects the build with the NERF_B200_DBG_* switches compiled in (libnerf_b200_exp.so: same sources,
-# -DNERF_B200_EXPERIMENTS; tools only)
-LIB_PATH = os.path.join(_HERE, "libnerf_b200_exp.so" if os.environ.get("NERF_B200_EXPERIMENTS") == "1" else "libnerf_b200.so")
+LIB_PATH = os.path.join(_HERE, "libnerf_b200.so")
 MAX_D = 16
 PREC_TC_FP16, PREC_FP32 = 0, 1
 
@@ -123,7 +121,6 @@ SIGNATURES = {
     "nerf_b200_timing_enable": (C.c_int, [C.c_int]),
     "nerf_b200_timing_read": (C.c_int, [C.POINTER(C.c_double), C.POINTER(C.c_int64), C.POINTER(C.c_double)]),
     "nerf_b200_timing_read_kinds": (C.c_int, [C.POINTER(C.c_double), C.POINTER(C.c_int64), C.POINTER(C.c_double), C.POINTER(C.c_double)]),
-    "nerf_b200_debug_set_trace": (C.c_int, [c_fp]),
 }
 
 # bring-up self-tests and micro-benchmarks: libnerf_b200_dev.so (include/nerf_b200_dev.h), never used by the product path

@@ -164,9 +164,6 @@ struct DgradParams {
   long long N; int S, rays_per_cta, nst_plan, D;
   uint32_t rec_mask, rec_grad;
   unsigned long long pair_half_bytes;       // bytes of one rank's half of the backward chunk stream
-  int dbg;                                  // NERF_B200_DBG_EMIT experiments (1: no record copies, 2: L2 evict_first hint)
-  unsigned long long* prof;                 // NERF_B200_DBG_DGRAD_PROF: per epilogue warp {total, waiting for d_full, waiting at the copy gates} cycles
-  int vc0, vc1;                             // forward CTAs [vc0, vc1) (both even): this launch's CTA b serves vc0 + b, vc0 + b + gridDim, ...
 };
 
 constexpr uint32_t DG2_SEED = SM_ENC;                                        // 131072: 32 KB, d_hv of ONE slot
@@ -214,10 +211,10 @@ dgrad_tc2_kernel(const DgradParams p, const __grid_constant__ CUtensorMap wmap, 
     }
   };
 
-  // rows: exactly the forward's split (forward CTA vc -> same rays -> same tile records).  The launch may be narrower than the
-  // forward's (gridDim even, so a pair keeps its ranks): each pair then walks the forward pairs b/2, b/2 + gridDim/2, ... --
-  // this is what lets the chain share the GPU with the weight-gradient kernel of the other pass (capi.cu).
-  const int D = p.D, NS = D + 1;
+  // rows: exactly the forward's split -- the launch has the forward's grid, and CTA vc serves forward CTA vc (same rays, same
+  // tile records)
+  const int vc = (int)blockIdx.x;
+  const int D = p.D, NS = D + 1, nst = plan_cta_nst(p.N, p.S, p.rays_per_cta, vc);
 
   for (int i = threadIdx.x; i < 256; i += TC_THREADS) s_alpha[i] = p.alpha_w[i];
   if (warp == 1 && lane == 0) {
@@ -240,8 +237,7 @@ dgrad_tc2_kernel(const DgradParams p, const __grid_constant__ CUtensorMap wmap, 
     // =========================== weight producer (both CTAs): this CTA's 8 KB half of every unit ===========
     uint32_t stage = 0, ph = 0;
     const int half_rows = (int)(p.pair_half_bytes >> 9);
-    for (int vc = p.vc0 + (int)blockIdx.x; vc < p.vc1; vc += (int)gridDim.x)
-    for (int st = 0, nst = plan_cta_nst(p.N, p.S, p.rays_per_cta, vc); st < nst; ++st) {
+    for (int st = 0; st < nst; ++st) {
       int row = (int)rank * half_rows;
       for (int j = 0; j < NS; ++j) {
         const int nu = bwd_step_units(j);
@@ -268,8 +264,7 @@ dgrad_tc2_kernel(const DgradParams p, const __grid_constant__ CUtensorMap wmap, 
     const uint64_t bdesc0 = ptx::umma_desc(sb, 512, ptx::UMMA_SW64);
     const uint32_t tmem0 = __shfl_sync(0xffffffffu, tmem, 0);
     const uint32_t idesc = ptx::umma_idesc_f16(256, 256);
-    for (int vc = p.vc0 + (int)blockIdx.x; vc < p.vc1; vc += (int)gridDim.x)
-    for (int st = 0, nst = plan_cta_nst(p.N, p.S, p.rays_per_cta, vc); st < nst; ++st) {
+    for (int st = 0; st < nst; ++st) {
       for (int j = 0; j < NS; ++j) {
         const int nu = bwd_step_units(j);
         for (int X = 0; X < 2; ++X) {
@@ -324,8 +319,7 @@ dgrad_tc2_kernel(const DgradParams p, const __grid_constant__ CUtensorMap wmap, 
     // the d_hv image (128 columns: in the record [half][K-block] pieces of 8 KB, in shared memory [K-block][half]) = four
     // 8 KB boxes of the gradient-record tensor map per (st, X); bytes of both CTAs are counted on the leader's barrier
     const int rec_rows = (int)(p.rec_grad >> 9);
-    for (int vc = p.vc0 + (int)blockIdx.x; vc < p.vc1; vc += (int)gridDim.x)
-    for (int st = 0, nst = plan_cta_nst(p.N, p.S, p.rays_per_cta, vc); st < nst; ++st) {
+    for (int st = 0; st < nst; ++st) {
       for (int X = 0; X < 2; ++X) {
         ptx::mbar_wait(bar_seedfree, (uint32_t)(X ^ 1));
         if (ptx::elect_one()) {
@@ -355,25 +349,19 @@ dgrad_tc2_kernel(const DgradParams p, const __grid_constant__ CUtensorMap wmap, 
     // as in the forward's training mode (fused_tc2.cuh)
     const uint32_t slice = (uint32_t)q * 4096u;
     const uint64_t l2_first = ptx::l2_policy_evict_first();
-    long long pf_gate = 0, pf_dfull = 0;
-    const long long pf_t0 = (kExp && p.prof) ? clock64() : 0;
     auto emit_gate = [&]() {
-      const long long c0 = (kExp && p.prof) ? clock64() : 0;
       if (lane == 0) ptx::bulk_wait_read1();
       __syncwarp();
-      if (kExp && p.prof) pf_gate += clock64() - c0;
     };
     auto emit_slice = [&](uint8_t* dst_img, int kb, uint32_t src_kblock) {
       ptx::fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) {
-        if (!(kExp && (p.dbg & 1))) ptx::bulk_s2g_hint(dst_img + img_slice_off(q, kb, 256), src_kblock + slice, 4096u, l2_first);
+        ptx::bulk_s2g_hint(dst_img + img_slice_off(q, kb, 256), src_kblock + slice, 4096u, l2_first);
         ptx::bulk_commit();
       }
     };
-    for (int vc = p.vc0 + (int)blockIdx.x; vc < p.vc1; vc += (int)gridDim.x) {
     const int nrows = plan_cta_rows(p.N, p.S, p.rays_per_cta, vc);
-    const int nst = plan_cta_nst(p.N, p.S, p.rays_per_cta, vc);
     const long long row_begin = (long long)vc * p.rays_per_cta * p.S;
     for (int st = 0; st < nst; ++st) {
       const int lr = st * TC_ST + X * TC_TILE + r;
@@ -386,9 +374,7 @@ dgrad_tc2_kernel(const DgradParams p, const __grid_constant__ CUtensorMap wmap, 
         // ReLU mask of this step's output (the pre-activation of pts layer D - j), fetched before the wait
         uint4 mk = make_uint4(0u, 0u, 0u, 0u);
         if (j >= 1) mk = *reinterpret_cast<const uint4*>(mrec + (uint32_t)(D - j) * 4096u + (uint32_t)ch * 2048u + (uint32_t)r * 16u);
-        { const long long c0 = (kExp && p.prof) ? clock64() : 0;
-          ptx::mbar_wait(bar_dfull + 8 * X, dph);
-          if (kExp && p.prof) pf_dfull += clock64() - c0; }
+        ptx::mbar_wait(bar_dfull + 8 * X, dph);
         dph ^= 1;
         ptx::tc_fence_after();
         const int colw = ch * 128;
@@ -431,12 +417,7 @@ dgrad_tc2_kernel(const DgradParams p, const __grid_constant__ CUtensorMap wmap, 
         emit_slice(grec + rec_grad_step(j), 2 * ch + 1, act_base + (uint32_t)(2 * ch + 1) * 16384u);
       }
     }
-    }
     if (lane == 0) ptx::bulk_wait_all();
-    if (kExp && p.prof && lane == 0) {
-      unsigned long long* o = p.prof + ((size_t)blockIdx.x * 16 + (warp - 4)) * 3;
-      o[0] = (unsigned long long)(clock64() - pf_t0); o[1] = (unsigned long long)pf_dfull; o[2] = (unsigned long long)pf_gate;
-    }
   }
 
   ptx::tc_fence_before();
@@ -469,9 +450,6 @@ struct WgradParams {
   const uint8_t* act; const uint8_t* grad; uint32_t rec_act, rec_grad;
   long long N; int S, rays_per_cta, nst_plan; long long n_tiles;
   const unsigned int* amax; float* partial; const float* d_raw; int njobs;
-  long long t0, t1;             // tiles [t0, t1) of the plan (a launch may cover part of a pass; the reduction adds up)
-  int dbg;                      // experiments (NERF_B200_DBG_WGRAD): 1 = no MMA (stream only; results are garbage)
-  unsigned long long* prof;     // experiments (NERF_B200_DBG_WGRAD_PROF): [CTA][2] globaltimer at start / end, or NULL
   WgradJob jobs[WG2_MAX_JOBS];
 };
 
@@ -480,7 +458,8 @@ __device__ __forceinline__ bool plan_tile_valid(const WgradParams& p, long long 
   return st < plan_cta_nst(p.N, p.S, p.rays_per_cta, cta);
 }
 
-// (launched as 2-CTA clusters only so that its CTAs fill whole TPCs: next to it the chain's CTA pairs need both SMs of a TPC)
+// (launched as 2-CTA clusters, so that its CTAs fill whole TPCs; launching it without clusters changes how its CTAs are
+// placed on the SMs and would need its own measurement)
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WG2_THREADS, 1) wgrad_tc_kernel(const WgradParams p) {
   uint8_t* smem = tc_smem;
   const uint32_t sb = ptx::smem_u32(smem);
@@ -488,10 +467,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WG2_THREADS, 1) wgra
   if ((sb & 1023u) != 0) __trap();
   int ji = -1;
   for (int i = 0; i < p.njobs; ++i) if ((int)blockIdx.x >= p.jobs[i].cta0 && (int)blockIdx.x < p.jobs[i].cta0 + p.jobs[i].ncta) ji = i;
-  if (kExp && p.prof && threadIdx.x == 0) { unsigned long long t_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_)); p.prof[2 * blockIdx.x] = t_; }
   if (ji < 0) return;                                   // (uniform per CTA, before any barrier / allocation)
   const WgradJob job = p.jobs[ji];
-  const int g = (int)blockIdx.x - job.cta0, G = job.ncta;
+  const long long g = (int)blockIdx.x - job.cta0, G = job.ncta;        // 64-bit, as the tile indices they step
   const uint32_t bar_full = sb + WG2_BARS, bar_empty = sb + WG2_BARS + 32, bar_done = sb + WG2_BARS + 64;
   uint32_t* s_tmem = reinterpret_cast<uint32_t*>(smem + WG2_BARS + 96);
   if (threadIdx.x == 0) {
@@ -510,11 +488,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WG2_THREADS, 1) wgra
   const uint32_t stride = (uint32_t)(xkb + ykb) * 8192u;
   const uint32_t nstg = (WG2_BARS / stride < (uint32_t)WG2_MAX_STAGES) ? WG2_BARS / stride : (uint32_t)WG2_MAX_STAGES;
   long long my_halves = 0;
-  for (long long t = p.t0 + g; t < p.t1; t += G) if (plan_tile_valid(p, t)) my_halves += 2;
+  for (long long t = g; t < p.n_tiles; t += G) if (plan_tile_valid(p, t)) my_halves += 2;
 
   if (warp == 4) {
     uint32_t s = 0, ph = 0;
-    for (long long t = p.t0 + g; t < p.t1; t += G) {
+    for (long long t = g; t < p.n_tiles; t += G) {
       if (!plan_tile_valid(p, t)) continue;
       for (int h = 0; h < 2; ++h) {
         ptx::mbar_wait(bar_empty + 8 * s, ph ^ 1);
@@ -523,14 +501,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WG2_THREADS, 1) wgra
           // 64-row half tile h of each operand: its K-blocks are adjacent in the record -> one contiguous piece per operand
           const uint8_t* xs = p.grad + (size_t)t * p.rec_grad + job.a_off + (size_t)h * xkb * 8192;
           const uint8_t* ys = p.act + (size_t)t * p.rec_act + job.b_off + (size_t)h * ykb * 8192;
-          if (kExp && (p.dbg & 2)) {
-            const uint64_t pol = ptx::l2_policy_evict_first();
-            ptx::bulk_g2s_hint(sb + s * stride, xs, (uint32_t)xkb * 8192u, bar_full + 8 * s, pol);
-            ptx::bulk_g2s_hint(sb + s * stride + ybase, ys, (uint32_t)ykb * 8192u, bar_full + 8 * s, pol);
-          } else {
           ptx::bulk_g2s(sb + s * stride, xs, (uint32_t)xkb * 8192u, bar_full + 8 * s);
           ptx::bulk_g2s(sb + s * stride + ybase, ys, (uint32_t)ykb * 8192u, bar_full + 8 * s);
-          }
         }
         __syncwarp();
         if (++s == nstg) { s = 0; ph ^= 1; }
@@ -543,9 +515,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WG2_THREADS, 1) wgra
     for (long long i = 0; i < my_halves; ++i) {
       ptx::mbar_wait(bar_full + 8 * s, ph);
       ptx::tc_fence_after();
-      if (kExp && (p.dbg & 1)) {
-        if (ptx::elect_one()) { ptx::mbar_arrive(bar_empty + 8 * s); if (i == my_halves - 1) ptx::mbar_arrive(bar_done); }
-      } else if (ptx::elect_one()) {
+      if (ptx::elect_one()) {
         const uint32_t xb = sb + s * stride, yb = xb + ybase;
         for (int mh = 0; mh < mhalves; ++mh)
 #pragma unroll
@@ -581,19 +551,18 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WG2_THREADS, 1) wgra
       return (lr_ < plan_cta_rows(p.N, p.S, p.rays_per_cta, cta_)) ? p.d_raw[((long long)cta_ * p.rays_per_cta * p.S + lr_) * 4 + 3] : 0.f;
     };
     auto next_valid = [&](long long t_) -> long long {
-      for (t_ += G; t_ < p.t1; t_ += G) if (plan_tile_valid(p, t_)) return t_;
+      for (t_ += G; t_ < p.n_tiles; t_ += G) if (plan_tile_valid(p, t_)) return t_;
       return -1;
     };
     int dslot = 0;
     if (job.aux == 2) {
-      long long t0 = p.t0 + g - G;
-      t0 = next_valid(t0);
+      const long long t0 = next_valid(g - G);
       const float v = (t0 >= 0) ? load_dsig(t0) : 0.f;
       s_dsig[tid] = v;
       bsum += v;
       ptx::named_bar_sync(1, 128);
     }
-    for (long long t = p.t0 + g; t < p.t1; t += G) {
+    for (long long t = g; t < p.n_tiles; t += G) {
       if (!plan_tile_valid(p, t)) continue;
       const int cta = (int)(t / (2 * p.nst_plan)), st = (int)((t >> 1) % p.nst_plan), X = (int)(t & 1);
       const int nrows = plan_cta_rows(p.N, p.S, p.rays_per_cta, cta);
@@ -718,7 +687,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WG2_THREADS, 1) wgra
   ptx::tc_fence_before();
   __syncthreads();
   if (warp == 0) ptx::tmem_dealloc(tmem, 512);
-  if (kExp && p.prof && threadIdx.x == 0) { unsigned long long t_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_)); p.prof[2 * blockIdx.x + 1] = t_; }
 }
 
 // dst[o][i] += inv_scale * sum_g partial[g][o][i]   (i < n_valid; dst row stride ldw)

@@ -8,7 +8,6 @@
 #include "fused_tc2.cuh"
 #include "bwd_tc2.cuh"
 #include "train_step.cuh"
-#include <stdlib.h>
 
 namespace nb {
 thread_local char g_err[512] = {0};
@@ -36,8 +35,6 @@ static double net_macs_per_row(const NerfNetParams& n) {
   return m;
 }
 
-static long long* g_trace = nullptr;      // debug: device buffer of 4096 int64 clock stamps (NERF_B200_TRACE builds)
-
 static int check_tc_net(const NerfNetParams* net) {
   NB_CHECK_ARG(net != nullptr, "net is NULL");
   NB_CHECK_ARG(net->W == TC_W, "tensor-core path supports netwidth == 256 (got %d); use precision=FP32", net->W);
@@ -55,9 +52,7 @@ static int smem_optin(const void* fn, size_t bytes) {
 
 // per-device facts (SM count; which kernels already have their > 48 KB shared-memory opt-in): the library may be used
 // on several devices of one process, and cudaFuncSetAttribute is per device
-static const char* exp_env(const char* name) { return kExp ? getenv(name) : nullptr; }      // experiment switches: product build ignores them
-static int dbg_emit() { static int v = -1; if (v < 0) { const char* e = exp_env("NERF_B200_DBG_EMIT"); v = e ? atoi(e) : 0; } return v; }
-struct DeviceState { int sms; bool optin_fwd, optin_bwd; cudaStream_t side; cudaEvent_t ev[10]; };
+struct DeviceState { int sms; bool optin_fwd, optin_bwd; cudaStream_t side; cudaEvent_t ev[4]; };
 static DeviceState* device_state() {
   static DeviceState st[64];
   static bool init[64] = {false};
@@ -73,7 +68,7 @@ static DeviceState* device_state() {
     // lazily inside a call that may be running under stream capture
     st[dev].side = nullptr;
     if (cudaStreamCreateWithFlags(&st[dev].side, cudaStreamNonBlocking) == cudaSuccess) {
-      for (int i = 0; i < 10; ++i)
+      for (int i = 0; i < 4; ++i)
         if (cudaEventCreateWithFlags(&st[dev].ev[i], cudaEventDisableTiming) != cudaSuccess) { cudaStreamDestroy(st[dev].side); st[dev].side = nullptr; break; }
     } else {
       st[dev].side = nullptr;
@@ -154,7 +149,6 @@ static int launch_march(const float* rays, int ray_stride, const float* z_vals, 
     if (int rc = smem_optin((const void*)march_tc2_kernel<true>, SM_ALLOC)) return rc;
     ds->optin_fwd = true;
   }
-  p.trace = g_trace;
   TrainSaveDev sv;
   memset(&sv, 0, sizeof(sv));
   if (save) {
@@ -165,7 +159,6 @@ static int launch_march(const float* rays, int ray_stride, const float* z_vals, 
     NB_CHECK_ARG((reinterpret_cast<uintptr_t>(save->act) & 15) == 0 && (reinterpret_cast<uintptr_t>(save->mask) & 15) == 0, "save buffers must be 16-byte aligned");
     sv.act = static_cast<uint8_t*>(save->act); sv.mask = static_cast<uint8_t*>(save->mask);
     sv.nst_plan = plan.nst; sv.rec_act = rec_act_bytes(net->D); sv.rec_mask = rec_mask_bytes(net->D);
-    sv.dbg = dbg_emit();
   }
   TimedLaunch* tl = nullptr;
   if (g_timing && g_ntimed < 4096) {
@@ -787,7 +780,7 @@ BwdTcJobs make_bwd_jobs(const NerfNetParams& n, const NerfNetGrads* g, int sms) 
     for (int i = 1; i < J.n; ++i) if (frac[i] > frac[b]) b = i;
     ++J.w[b].ncta; ++used; frac[b] -= 1.0;
   }
-  while (used > sms) {                               // (tiny launches: more jobs than CTAs is rejected by the caller's minimum)
+  while (used > sms) {                               // (only where the GPU has few SMs for the number of jobs)
     int b = 0;
     for (int i = 1; i < J.n; ++i) if (J.w[i].ncta > J.w[b].ncta) b = i;
     --J.w[b].ncta; --used;
@@ -846,9 +839,9 @@ int nerf_b200_march_bwd_tc_layout(int64_t N, int S, const NerfNetParams* net, in
 }
 
 namespace {
-// One pass of the tensor-core backward, split into its phases so that the two passes of render_rays can interleave: the data-
-// gradient chain is bound by HBM WRITES (3.9 TB/s ceiling), the weight gradient by HBM READS; side by side on disjoint SMs they
-// share a bus that carries 6.6 TB/s of mixed traffic (profiles/r02_hbm_probe.json).
+// One pass of the tensor-core backward, split into its phases so that the two passes of render_rays can interleave: the small
+// kernels of one pass (prologue, heads) run on a side stream next to the other pass's big kernels (dgrad, wgrad), which each
+// take the whole GPU.  run() is the pass on one stream.
 struct BwdTcPass {
   const float* rays; const float* z; const float* noise; int64_t N; int S; const NerfNetParams* net; const void* packed;
   const NerfRenderCfg* cfg; const float* raw; const NerfTrainSave* save; const float* g_rgb; const NerfNetGrads* grads;
@@ -901,8 +894,8 @@ struct BwdTcPass {
     return 0;
   }
 
-  // 3. dgrad chain of the forward's CTAs [vc0, vc1) on at most `ctas` CTAs (CTA pairs, the forward's tile order)
-  int dgrad(cudaStream_t st, int ctas, int vc0, int vc1) {
+  // 3. dgrad chain: the forward's grid (CTA pairs), CTA b serves the tiles of forward CTA b
+  int dgrad(cudaStream_t st) {
     const int D = net->D;
     const uint8_t* pk = static_cast<const uint8_t*>(packed);
     DgradParams dp;
@@ -910,11 +903,6 @@ struct BwdTcPass {
     dp.N = N; dp.S = S; dp.rays_per_cta = plan.rays_per_cta; dp.nst_plan = plan.nst; dp.D = D;
     dp.rec_mask = rec_mask_bytes(D); dp.rec_grad = rec_grad_bytes(D);
     dp.pair_half_bytes = PL.bwd_bytes / 2;
-    dp.vc0 = vc0; dp.vc1 = vc1; dp.dbg = dbg_emit();
-    int grid = vc1 - vc0;
-    if (grid > ctas) grid = ctas;
-    grid &= ~1;
-    if (grid < 2) grid = 2;
     CUtensorMap wmap, gmap;
     NB_TRY(make_row_map(&wmap, pk + PL.off_bwd_pair, PL.bwd_bytes, 16));
     NB_TRY(make_row_map(&gmap, grec, (size_t)plan.n_tiles * rec_grad_bytes(D), 16));      // 8 KB boxes: the pieces of the d_hv image
@@ -922,81 +910,40 @@ struct BwdTcPass {
     if (g_timing && g_ntimed < 4096) {
       tl = &g_timed[g_ntimed++];
       cudaEventCreate(&tl->a); cudaEventCreate(&tl->b);
-      tl->flops = 2.0 * ((double)(net->W / 2) * net->W + (double)D * net->W * net->W) * (double)(N * (long long)S) * (double)(vc1 - vc0) / (double)plan.grid;
+      tl->flops = 2.0 * ((double)(net->W / 2) * net->W + (double)D * net->W * net->W) * (double)(N * (long long)S);
       tl->kind = 1;
       cudaEventRecord(tl->a, st);
     }
-    static const char* prof_path = exp_env("NERF_B200_DBG_DGRAD_PROF");     // experiments: where the epilogue warps wait
-    static unsigned long long* prof_dev = nullptr;
-    dp.prof = nullptr;
-    if (prof_path) { if (!prof_dev) NB_CUDA(cudaMalloc(&prof_dev, 512 * 16 * 3 * 8)); dp.prof = prof_dev; }
-    dgrad_tc2_kernel<<<grid, TC_THREADS, SM_ALLOC, st>>>(dp, wmap, gmap);
+    dgrad_tc2_kernel<<<plan.grid, TC_THREADS, SM_ALLOC, st>>>(dp, wmap, gmap);
     if (tl) cudaEventRecord(tl->b, st);
     NB_LAUNCH_OK("dgrad_tc2_kernel");
-    if (prof_path) {
-      static unsigned long long h[512 * 16 * 3];
-      NB_CUDA(cudaStreamSynchronize(st));
-      NB_CUDA(cudaMemcpy(h, prof_dev, (size_t)grid * 16 * 3 * 8, cudaMemcpyDeviceToHost));
-      if (FILE* f = fopen(prof_path, "a")) {
-        double tot = 0, df = 0, gt = 0;
-        for (int i = 0; i < grid * 16; ++i) { tot += (double)h[3 * i]; df += (double)h[3 * i + 1]; gt += (double)h[3 * i + 2]; }
-        fprintf(f, "dgrad S=%d grid=%d: epilogue warps, mean cycles: total %.0f, waiting for d_full %.0f (%.1f %%), at the copy gates %.0f (%.1f %%)\n", S, grid,
-                tot / (grid * 16), df / (grid * 16), 100.0 * df / tot, gt / (grid * 16), 100.0 * gt / tot);
-        fclose(f);
-      }
-    }
     return 0;
   }
 
-  // 4. weight gradients (layer-major) + bias gradients of the forward's CTAs [vc0, vc1) on `ctas` CTAs, then the reduction of
-  // the per-CTA partial blocks (adds into the gradient tensors, so a pass may be covered by several launches)
-  int wgrad(cudaStream_t st, int ctas, int vc0, int vc1) {
+  // 4. weight gradients (layer-major) + bias gradients on all SMs, then the reduction of the per-CTA partial blocks (adds
+  // into the gradient tensors)
+  int wgrad(cudaStream_t st) {
     const int D = net->D;
-    BwdTcJobs J = make_bwd_jobs(*net, grads, ctas & ~1);           // whole CTA pairs: the kernel launches as 2-CTA clusters
+    BwdTcJobs J = make_bwd_jobs(*net, grads, ds->sms & ~1);        // whole CTA pairs: the kernel launches as 2-CTA clusters
     J.w[0].aux = 1; J.w[0].aux_dst = dsum;            // views job: per-ray row sums of d_hv
     J.w[1].aux = 2; J.w[1].aux_dst = grads->alpha_w; J.w[1].aux_b = grads->alpha_b;   // feature job: alpha_linear gradients
-    { static int noaux = -1; if (noaux < 0) { const char* e = exp_env("NERF_B200_DBG_NOAUX"); noaux = e ? atoi(e) : 0; }
-      if (noaux & 1) J.w[0].aux = 0;
-      if (noaux & 2) J.w[1].aux = 0;
-      if (noaux & 4) for (int i = 0; i < J.n; ++i) J.w[i].db = nullptr; }
     WgradParams wp;
     memset(&wp, 0, sizeof(wp));
     wp.act = act; wp.grad = grec; wp.rec_act = rec_act_bytes(D); wp.rec_grad = rec_grad_bytes(D);
     wp.N = N; wp.S = S; wp.rays_per_cta = plan.rays_per_cta; wp.nst_plan = plan.nst; wp.n_tiles = plan.n_tiles;
-    wp.t0 = (long long)vc0 * plan.nst * 2; wp.t1 = (long long)vc1 * plan.nst * 2;
     wp.amax = amax; wp.partial = partial; wp.d_raw = d_raw; wp.njobs = J.n;
-    { static int wd = -1; if (wd < 0) { const char* e = exp_env("NERF_B200_DBG_WGRAD"); wd = e ? atoi(e) : 0; } wp.dbg = wd; }
     for (int i = 0; i < J.n; ++i) wp.jobs[i] = J.w[i];
     TimedLaunch* tl = nullptr;
     if (g_timing && g_ntimed < 4096) {
       tl = &g_timed[g_ntimed++];
       cudaEventCreate(&tl->a); cudaEventCreate(&tl->b);
-      tl->flops = 2.0 * (net_macs_per_row(*net) - (double)net->W - 3.0 * (net->W / 2) - (double)net->input_ch_views * (net->W / 2)) * (double)(N * (long long)S) * (double)(vc1 - vc0) / (double)plan.grid;
+      tl->flops = 2.0 * (net_macs_per_row(*net) - (double)net->W - 3.0 * (net->W / 2) - (double)net->input_ch_views * (net->W / 2)) * (double)(N * (long long)S);
       tl->kind = 2;
       cudaEventRecord(tl->a, st);
     }
-    static const char* prof_path = exp_env("NERF_B200_DBG_WGRAD_PROF");     // experiments: per-CTA start / end times appended to a file
-    static unsigned long long* prof_dev = nullptr;
-    if (prof_path) { if (!prof_dev) NB_CUDA(cudaMalloc(&prof_dev, 1024 * 16)); wp.prof = prof_dev; }
     wgrad_tc_kernel<<<J.total_ctas, WG2_THREADS, WG2_TOTAL, st>>>(wp);
     if (tl) cudaEventRecord(tl->b, st);
     NB_LAUNCH_OK("wgrad_tc_kernel");
-    if (prof_path) {
-      unsigned long long h[2048];
-      NB_CUDA(cudaStreamSynchronize(st));
-      NB_CUDA(cudaMemcpy(h, prof_dev, (size_t)J.total_ctas * 16, cudaMemcpyDeviceToHost));
-      if (FILE* f = fopen(prof_path, "a")) {
-        unsigned long long t0 = ~0ull;
-        for (int i = 0; i < J.total_ctas; ++i) if (h[2 * i] < t0) t0 = h[2 * i];
-        fprintf(f, "launch S=%d ctas=%d\n", S, J.total_ctas);
-        for (int j = 0; j < J.n; ++j) {
-          unsigned long long lo = ~0ull, hi = 0;
-          for (int i = J.w[j].cta0; i < J.w[j].cta0 + J.w[j].ncta; ++i) { if (h[2 * i + 1] - t0 < lo) lo = h[2 * i + 1] - t0; if (h[2 * i + 1] - t0 > hi) hi = h[2 * i + 1] - t0; }
-          fprintf(f, "  job %2d Mc=%3d Nc=%3d aux=%d db=%d ctas=%2d end_us min %.1f max %.1f\n", j, J.w[j].Mc, J.w[j].Nc, J.w[j].aux, J.w[j].db != nullptr, J.w[j].ncta, lo * 1e-3, hi * 1e-3);
-        }
-        fclose(f);
-      }
-    }
     ReduceParams rp;
     memset(&rp, 0, sizeof(rp));
     rp.partial = partial; rp.amax = amax; rp.njobs = J.n;
@@ -1019,6 +966,14 @@ struct BwdTcPass {
     views_feat_wgrad_kernel<<<128, 256, 0, st>>>(gv, dbv, net->feature_w, net->feature_b, grads->views_w, net->W + ICV);
     NB_LAUNCH_OK("views_feat_wgrad_kernel");
     return 0;
+  }
+
+  // the whole pass on one stream
+  int run(cudaStream_t st) {
+    NB_TRY(prologue(st));
+    NB_TRY(dgrad(st));
+    NB_TRY(wgrad(st));
+    return heads(st);
   }
 };
 
@@ -1049,11 +1004,7 @@ int nerf_b200_march_bwd_tc(const float* rays, const float* z_vals, const float* 
   cudaStream_t st = (cudaStream_t)stream;
   BwdTcPass b = bind_pass(rays, N, cfg, &q);
   NB_TRY(b.init(workspace, workspace_bytes));
-  NB_TRY(b.prologue(st));
-  NB_TRY(b.dgrad(st, b.plan.grid, 0, b.plan.grid));
-  NB_TRY(b.wgrad(st, b.ds->sms, 0, b.plan.grid));
-  NB_TRY(b.heads(st));
-  return 0;
+  return b.run(st);
 }
 
 size_t nerf_b200_render_rays_bwd_tc_workspace_bytes(int64_t N, int S_coarse, const NerfNetParams* net_coarse, int S_fine, const NerfNetParams* net_fine) {
@@ -1067,13 +1018,13 @@ size_t nerf_b200_render_rays_bwd_tc_workspace_bytes(int64_t N, int S_coarse, con
 }
 
 // Backward of both passes of render_rays (run_nerf.py:765-772: loss = img2mse(rgb) + img2mse(rgb0); z_samples is detached, :394,
-// so the passes are independent).  Two streams (graph-capturable: the side stream forks from and joins `stream`).  Default schedule:
+// so the passes are independent).  Two streams (graph-capturable: the side stream forks from and joins `stream`):
 //   main: prologue(c) dgrad(c) | wgrad(c)      | dgrad(f) | wgrad(f) heads(f) |
 //   side:                      | prologue(f)   |          | heads(c)          | join
 // the small memory-bound kernels of one pass (compositing adjoint, seed tiles + rgb_linear, view-column gradients) run on the SM
 // resources the weight-gradient kernel leaves free (it holds one 192-thread CTA per SM) instead of between the big kernels.
-// NERF_B200_BWD_OVERLAP = "0": one stream, one pass after the other;  "w[,chunks]" (w >= 16): split the SMs -- the fine pass's chain
-// on sms - w of them next to a weight gradient on w (measured slower in every split: profiles/r02_bwd_overlap_sweep.jsonl).
+// One stream, one pass after the other: a single pass, one network serving both passes (its gradients would race), a fine
+// pass of fewer than 4 CTAs, or no side stream (its creation failed).
 int nerf_b200_render_rays_bwd_tc(const float* rays, int64_t N, const NerfRenderCfg* cfg, const NerfBwdPass* coarse, const NerfBwdPass* fine,
                                  void* workspace, size_t workspace_bytes, void* stream) {
   if (int rc = check_bwd_pass(rays, coarse, cfg)) return rc;
@@ -1084,86 +1035,32 @@ int nerf_b200_render_rays_bwd_tc(const float* rays, int64_t N, const NerfRenderC
   const size_t cb = bwd_pass_bytes(N, coarse->S, coarse->net);
   NB_CHECK_ARG(workspace && workspace_bytes >= cb, "render_rays_bwd_tc workspace too small");
   NB_TRY(c.init(workspace, cb));
-  DeviceState* ds = c.ds;
-  const int sms = ds->sms;
-  static int env_w = -2, env_chunks = 1;                // -1: default schedule
-  if (env_w == -2) {
-    const char* e = getenv("NERF_B200_BWD_OVERLAP");
-    env_w = -1;
-    if (e) { int a = -1, k = 1; const int n = sscanf(e, "%d,%d", &a, &k); if (n >= 1) env_w = a; if (n >= 2 && k > 0) env_chunks = k; }
-  }
-  if (!fine) {
-    NB_TRY(c.prologue(st)); NB_TRY(c.dgrad(st, c.plan.grid, 0, c.plan.grid)); NB_TRY(c.wgrad(st, sms, 0, c.plan.grid)); NB_TRY(c.heads(st));
-    return 0;
-  }
+  if (!fine) return c.run(st);
   BwdTcPass f = bind_pass(rays, N, cfg, fine);
   NB_TRY(f.init(static_cast<uint8_t*>(workspace) + cb, workspace_bytes - cb));
-  const bool shared_grads = (coarse->grads->pts_w[0] == fine->grads->pts_w[0]);       // one network serving both passes: += races
-  int w = env_w;
-  if (w > sms - 16) w = sms - 16;
-  if (w > 0) w &= ~1;
-  if (w == 0 || (w > 0 && w < 16) || shared_grads || f.plan.grid < 4) {
-    static int dc = -1, wc = -1;                       // NERF_B200_DBG_BWD_CTAS="d,w": CTA caps of the two kernels (scaling experiments)
-    if (dc < 0) { dc = 1 << 20; wc = sms; const char* e = exp_env("NERF_B200_DBG_BWD_CTAS"); if (e) { int a = 0, b = 0; if (sscanf(e, "%d,%d", &a, &b) == 2 && a >= 2 && b >= 16 && b <= sms) { dc = a; wc = b; } } }
-    NB_TRY(c.prologue(st)); NB_TRY(c.dgrad(st, dc, 0, c.plan.grid)); NB_TRY(c.wgrad(st, wc, 0, c.plan.grid)); NB_TRY(c.heads(st));
-    NB_TRY(f.prologue(st)); NB_TRY(f.dgrad(st, dc, 0, f.plan.grid)); NB_TRY(f.wgrad(st, wc, 0, f.plan.grid)); NB_TRY(f.heads(st));
-    return 0;
-  }
-  if (!ds->side) {                                   // (creation failed at start-up: one stream, one pass after the other)
-    NB_TRY(c.prologue(st)); NB_TRY(c.dgrad(st, c.plan.grid, 0, c.plan.grid)); NB_TRY(c.wgrad(st, sms, 0, c.plan.grid)); NB_TRY(c.heads(st));
-    NB_TRY(f.prologue(st)); NB_TRY(f.dgrad(st, f.plan.grid, 0, f.plan.grid)); NB_TRY(f.wgrad(st, sms, 0, f.plan.grid)); NB_TRY(f.heads(st));
-    return 0;
+  DeviceState* ds = c.ds;
+  const bool shared_grads = (coarse->grads->pts_w[0] == fine->grads->pts_w[0]);
+  if (shared_grads || f.plan.grid < 4 || !ds->side) {
+    NB_TRY(c.run(st));
+    return f.run(st);
   }
   cudaStream_t sd = ds->side;
-  if (w < 0) {
-    // ---- default: the small kernels ride next to the weight-gradient kernels ----
-    NB_TRY(c.prologue(st));
-    NB_TRY(c.dgrad(st, c.plan.grid, 0, c.plan.grid));
-    NB_CUDA(cudaEventRecord(ds->ev[0], st));
-    NB_CUDA(cudaStreamWaitEvent(sd, ds->ev[0], 0));
-    NB_TRY(f.prologue(sd));
-    NB_CUDA(cudaEventRecord(ds->ev[1], sd));
-    NB_TRY(c.wgrad(st, sms, 0, c.plan.grid));
-    NB_CUDA(cudaStreamWaitEvent(st, ds->ev[1], 0));
-    NB_TRY(f.dgrad(st, f.plan.grid, 0, f.plan.grid));
-    NB_CUDA(cudaEventRecord(ds->ev[2], st));
-    NB_CUDA(cudaStreamWaitEvent(sd, ds->ev[2], 0));
-    NB_TRY(c.heads(sd));
-    NB_CUDA(cudaEventRecord(ds->ev[3], sd));
-    NB_TRY(f.wgrad(st, sms, 0, f.plan.grid));
-    NB_TRY(f.heads(st));
-    NB_CUDA(cudaStreamWaitEvent(st, ds->ev[3], 0));
-    return 0;
-  }
-  // ---- SM split (experiment) ----
-  int chunks = env_chunks;
-  if (chunks > 8) chunks = 8;
-  if (chunks > f.plan.grid / 2) chunks = f.plan.grid / 2;
-  if (chunks < 1) chunks = 1;
   NB_TRY(c.prologue(st));
-  NB_TRY(f.prologue(st));
-  NB_TRY(c.dgrad(st, c.plan.grid, 0, c.plan.grid));
+  NB_TRY(c.dgrad(st));
   NB_CUDA(cudaEventRecord(ds->ev[0], st));
   NB_CUDA(cudaStreamWaitEvent(sd, ds->ev[0], 0));
-  NB_TRY(c.wgrad(sd, w, 0, c.plan.grid));
+  NB_TRY(f.prologue(sd));
+  NB_CUDA(cudaEventRecord(ds->ev[1], sd));
+  NB_TRY(c.wgrad(st));
+  NB_CUDA(cudaStreamWaitEvent(st, ds->ev[1], 0));
+  NB_TRY(f.dgrad(st));
+  NB_CUDA(cudaEventRecord(ds->ev[2], st));
+  NB_CUDA(cudaStreamWaitEvent(sd, ds->ev[2], 0));
   NB_TRY(c.heads(sd));
-  // fine pass: `chunks` ranges of the forward's CTA pairs; chunk k's weight gradient runs on the side stream next to chunk
-  // k + 1's chain, the last chunk's on the main stream with all SMs
-  const int pairs = f.plan.grid / 2;
-  int v0 = 0, v1 = 0;
-  for (int k = 0; k < chunks; ++k) {
-    v0 = 2 * (int)((long long)pairs * k / chunks); v1 = 2 * (int)((long long)pairs * (k + 1) / chunks);
-    NB_TRY(f.dgrad(st, sms - w, v0, v1));
-    if (k + 1 < chunks) {
-      NB_CUDA(cudaEventRecord(ds->ev[k + 1], st));
-      NB_CUDA(cudaStreamWaitEvent(sd, ds->ev[k + 1], 0));
-      NB_TRY(f.wgrad(sd, w, v0, v1));
-    }
-  }
-  NB_CUDA(cudaEventRecord(ds->ev[9], sd));
-  NB_CUDA(cudaStreamWaitEvent(st, ds->ev[9], 0));
-  NB_TRY(f.wgrad(st, sms, v0, v1));
+  NB_CUDA(cudaEventRecord(ds->ev[3], sd));
+  NB_TRY(f.wgrad(st));
   NB_TRY(f.heads(st));
+  NB_CUDA(cudaStreamWaitEvent(st, ds->ev[3], 0));
   return 0;
 }
 
@@ -1189,7 +1086,5 @@ int nerf_b200_adam_step(float* params, const float* grads, float* exp_avg, float
   NB_LAUNCH_OK("adam_advance_kernel");
   return 0;
 }
-
-int nerf_b200_debug_set_trace(void* dev_buf_4096_i64) { g_trace = static_cast<long long*>(dev_buf_4096_i64); return 0; }
 
 }  // extern "C"

@@ -301,8 +301,6 @@ struct MarchParams {
   int white_bkgd, do_composite;
   NerfPassOut out;
   unsigned long long pair_half_bytes;     // pair kernel: bytes of one rank's half of the chunk stream
-  long long* trace;                       // debug: clock64 timestamps of CTA 0, super-tile 1 (or NULL)
-  int dbg;                                // debug: NERF_B200_DBG bit flags for A/B experiments (0 in production)
 };
 
 // compositing carry of the ray that is still open at a warp boundary (shared memory, 32 B)

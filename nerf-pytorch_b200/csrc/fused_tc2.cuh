@@ -40,14 +40,9 @@ constexpr uint32_t P2_HEADS = P2_BIASB + TC_BIAS_CHUNK_BYTES / 2;     // 225792:
 constexpr uint32_t P2_BARS = P2_HEADS + 4128;                         // 229920: mbarriers
 constexpr uint32_t P2_MISC = P2_BARS + 256;                           // 230176: tmem ptr, compositing carry, pass counter
 constexpr uint32_t P2_TOTAL = P2_MISC + 128;                          // 230304
-#ifdef NERF_B200_TRACE
-constexpr bool kTrace2 = true;       // clock64 / heartbeat hooks (tools/trace_march.py); compiled out by default
-#else
-constexpr bool kTrace2 = false;
-#endif
 
 // training-mode save buffers of one pass (train_common.cuh)
-struct TrainSaveDev { uint8_t* act; uint8_t* mask; int nst_plan; uint32_t rec_act, rec_mask; int dbg; };   // dbg: NERF_B200_DBG_EMIT experiments
+struct TrainSaveDev { uint8_t* act; uint8_t* mask; int nst_plan; uint32_t rec_act, rec_mask; };
 static_assert(P2_TOTAL <= SM_ALLOC, "pair kernel shared-memory map exceeds the allocation");
 
 // ring units per pass of layer l (all even)
@@ -78,8 +73,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) march
   const uint32_t bar_encfull = sb + P2_BARS + 144;    //     (leader)
   const uint32_t bar_encfree = sb + P2_BARS + 152;
   // arrive on a barrier that lives in the leader CTA
-  // debug heartbeat: trace[blockIdx.x * 32 + role] = last wait this role entered (trace may be mapped host memory)
-  auto hb_ = [&](int role, long long code) { if (kTrace2 && p.trace && lane == 0 && blockIdx.x < 32) { volatile long long* t = p.trace; t[3000 + blockIdx.x * 32 + role] = code; } };
   // One arrival per warp; every lane has fenced its own writes (fence.proxy.async) before the __syncwarp.  The peer's
   // data is consumed by the peer SM's own tensor core, so the remote arrive needs no cluster-scope release.
   auto arrive_leader = [&](uint32_t bar) {
@@ -141,7 +134,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) march
         for (int X = 0; X < 2; ++X) {                               // pass of slot A, then the same units again for slot B
           int prow = row;
           for (int u = 0; u < nu; ++u) {
-            hb_(0, 1000000 + st * 10000 + l * 100 + X * 50 + u);
             ptx::mbar_wait(bar_wempty + 8 * stage, ph ^ 1);
             if (ptx::elect_one()) {
               // every load (cta_group::2) counts its bytes on the LEADER's w_full, which expects both CTAs' boxes
@@ -170,11 +162,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) march
     const uint64_t bias_desc = ptx::umma_desc(sb + P2_BIASB, 256, ptx::UMMA_SW32);
     const uint32_t tmem0 = __shfl_sync(0xffffffffu, tmem, 0);
     for (int st = 0; st < nst; ++st) {
-      const bool tr = kTrace2 && p.trace && blockIdx.x == 0 && st == 1;
-      const bool trs = kTrace2 && p.trace && blockIdx.x == 0 && lane == 0 && st < 48;
-      if (trs) p.trace[2200 + 2 * st] = clock64();
       ptx::mbar_wait_cluster(bar_encfull, st & 1);
-      if (trs) p.trace[2201 + 2 * st] = clock64();
       for (int l = 0; l < NL; ++l) {
         const int nu = tc2_layer_units(l, D, p.skip);
         const bool view_layer = (l == D + 1);
@@ -184,15 +172,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) march
         for (int X = 0; X < 2; ++X) {
           const uint32_t d_tmem = tmem0 + X * 256;
           const uint64_t sel_desc = ptx::umma_desc(sb + P2_ONES + X * 256, 0, ptx::UMMA_SW32);
-          long long* trp = p.trace + 4 * (l * 2 + X);          // pass trace: start, act seen, first MMA issued, pass issued
-          long long t_a = 0, t_b = 0, t_c = 0;
-          if (tr) t_a = clock64();
-          hb_(1, 4000000 + st * 10000 + l * 100 + X * 50);
           // slot X's accumulator drained and its A tile written by both CTAs' epilogue warps
           if (X == 0) { ptx::mbar_wait_cluster(bar_act, actph0); actph0 ^= 1; }
           else { ptx::mbar_wait_cluster(bar_act + 8, actph1); actph1 ^= 1; }
-          if (tr) t_b = clock64();
-          hb_(1, 5000000 + st * 10000 + l * 100 + X * 50);
           ptx::tc_fence_after();
           if (ptx::elect_one()) {
             // Everything between two MMAs of the issuing thread is exposed tensor-pipe idle time (the queue is
@@ -213,7 +195,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) march
                 acc = 1u;
                 if (c == 1 && l == last_enc_layer) ptx::mma2_commit_mc(bar_encfree, 3);
                 ptx::mma2_commit_mc(bar_wempty + 8 * s_, 3);
-                if (c == 0 && tr) t_c = clock64();
                 if (++s_ == TC2_NST) { s_ = 0; ph_ ^= 1; }
               }
             }
@@ -228,7 +209,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) march
                 ptx::mma2_f16_ss(d_tmem, ad + 2, bd + 2, idesc, 1u);
                 acc = 1u;
                 ptx::mma2_commit_mc(bar_wempty + 8 * s_, 3);
-                if (kc == 0 && tr && !skip_layer) t_c = clock64();
                 if (++s_ == TC2_NST) { s_ = 0; ph_ ^= 1; }
               }
             } else if (view_layer) {
@@ -245,12 +225,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) march
                   acc = 1u;
                 }
                 ptx::mma2_commit_mc(bar_wempty + 8 * s_, 3);
-                if (u == 0 && tr) t_c = clock64();
                 if (++s_ == TC2_NST) { s_ = 0; ph_ ^= 1; }
               }
             }
             ptx::mma2_commit_mc(bar_dfull + 8 * X, 3);
-            if (tr) { trp[0] = t_a; trp[1] = t_b; trp[2] = t_c; trp[3] = clock64(); }
           }
           __syncwarp();
           stage += (uint32_t)nu;
@@ -297,17 +275,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) march
     const uint32_t slice = (uint32_t)q * 4096u;
     const uint64_t l2_first = EMIT ? ptx::l2_policy_evict_first() : 0ull;      // records are written once, read once by the backward
     auto emit_gate = [&](bool all) {
-      if (kExp && (sv.dbg & 8)) return;
       if (lane == 0) { if (all) ptx::bulk_wait_read0(); else ptx::bulk_wait_read1(); }
       __syncwarp();
     };
     // dst_img: the image in the record, kb: its K-block, C: its columns; src_kblock: the K-block in shared memory
     auto emit_slice = [&](uint8_t* dst_img, int kb, int C, uint32_t src_kblock) {
-      if (kExp && (sv.dbg & 8)) return;
       ptx::fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) {
-        if (!(kExp && (sv.dbg & 1))) ptx::bulk_s2g_hint(dst_img + img_slice_off(q, kb, C), src_kblock + slice, 4096u, l2_first);
+        ptx::bulk_s2g_hint(dst_img + img_slice_off(q, kb, C), src_kblock + slice, 4096u, l2_first);
         ptx::bulk_commit();
       }
     };
@@ -322,13 +298,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) march
       if (n_ray > p.N - 1) n_ray = p.N - 1;                       // (padding CTA of an odd pair / empty range)
       if (n_ray < 0) n_ray = 0;
       for (int l = 0; l < NL; ++l) {
-        const bool tr = kTrace2 && p.trace && blockIdx.x == 0 && st == 1 && e == 0 && lane == 0;
-        long long* trp = p.trace + 2048 + 4 * (X * 16 + l);
-        if (tr) trp[0] = clock64();
         ptx::mbar_wait(bar_dfull + 8 * X, dph);
         dph ^= 1;
         ptx::tc_fence_after();
-        if (tr) trp[1] = clock64();
         if (l <= D) {
           // pts layer (ReLU) or feature layer (no activation): 128 columns per warp in 4 batches,
           // the TMEM load of batch b+1 in flight while batch b is converted and stored
@@ -347,7 +319,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) march
             if (b < 3) ptx::tmem_ld_x32(t_lane + col0 + 32, vn);
             float x[32];
             as_float32(v, x);
-            if (EMIT && l < D && !(kExp && (sv.dbg & 4))) {
+            if (EMIT && l < D) {
 #pragma unroll
               for (int j = 0; j < 32; ++j) mk[b] = mask_push(mk[b], x[j]);
             }
@@ -399,15 +371,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) march
           }
           ptx::tc_fence_before();
           ptx::fence_proxy_async_smem();
-          const long long t_f = (kTrace2 && p.trace && blockIdx.x < 2 && st == 1 && l == 3 && lane == 0) ? clock64() : 0;
           arrive_leader(bar_act + 8 * X);
           if (EMIT) {
-            if (l < D && !(kExp && (sv.dbg & 4))) *reinterpret_cast<uint4*>(mrec + (uint32_t)l * 4096u + (uint32_t)ch * 2048u + (uint32_t)r * 16u) = make_uint4(mk[0], mk[1], mk[2], mk[3]);
+            if (l < D) *reinterpret_cast<uint4*>(mrec + (uint32_t)l * 4096u + (uint32_t)ch * 2048u + (uint32_t)r * 16u) = make_uint4(mk[0], mk[1], mk[2], mk[3]);
             // second K-block of h_l (feature_linear's output, l == D, is not recorded)
             if (l < D && write_act) emit_slice(arec + rec_act_h(l), 2 * ch + 1, 256, act_base + (uint32_t)(2 * ch + 1) * 16384u);
           }
-          if (tr) trp[2] = clock64();
-          if (kTrace2 && p.trace && blockIdx.x < 2 && st == 1 && l == 3 && lane == 0) { p.trace[2500 + blockIdx.x * 32 + (warp - 4) * 2] = t_f; p.trace[2501 + blockIdx.x * 32 + (warp - 4) * 2] = clock64(); }
         } else {
           // views_linears[0] (N=128): 64 columns per warp; + per-ray view bias, ReLU, rgb_linear
           const float* vbrow = p.vb + n_ray * 128;
@@ -475,10 +444,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) march
     // =========================== sampler (warp 3) ===========================
     const int t = threadIdx.x - 96;                               // 0..31
     for (int st = 0; st < nst; ++st) {
-      const bool trs = kTrace2 && p.trace && blockIdx.x == 0 && t == 0 && st < 48;
-      if (trs) p.trace[2300 + 2 * st] = clock64();
       ptx::mbar_wait(bar_encfree, (st & 1) ^ 1);
-      if (trs) p.trace[2301 + 2 * st] = clock64();
       if (EMIT) { if (t == 0) ptx::bulk_wait_read0(); __syncwarp(); }   // the previous super-tile's encodings have been copied out
 #pragma unroll 1
       for (int i = 0; i < 8; ++i) {
@@ -505,13 +471,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) march
           ptx::bulk_s2g(sv.act + (size_t)((blockIdx.x * sv.nst_plan + st) * 2 + X) * sv.rec_act, sb + SM_ENC + X * 16384, 16384u);
         ptx::bulk_commit();
       }
-      if (trs) p.trace[2400 + st] = clock64();
     }
     if (EMIT && t == 0) ptx::bulk_wait_all();
   }
 
-
-  hb_(warp, 7000000);
   ptx::tc_fence_before();
   __syncthreads();
   ptx::cluster_sync();                                  // the pair's MMAs / multicast commits are all done

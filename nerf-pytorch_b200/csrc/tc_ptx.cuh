@@ -53,10 +53,6 @@ __device__ __forceinline__ uint64_t l2_policy_evict_first() {
 __device__ __forceinline__ void bulk_s2g_hint(void* dst_gmem, uint32_t src_smem, uint32_t bytes, uint64_t policy) {
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(dst_gmem), "r"(src_smem), "r"(bytes), "l"(policy) : "memory");
 }
-__device__ __forceinline__ void bulk_g2s_hint(uint32_t dst_smem, const void* src_gmem, uint32_t bytes, uint32_t bar, uint64_t policy) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;"
-               ::"r"(dst_smem), "l"(src_gmem), "r"(bytes), "r"(bar), "l"(policy) : "memory");
-}
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 // all of this thread's committed groups have finished READING shared memory (the source may be overwritten)
 __device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }

@@ -30,16 +30,6 @@
 
 namespace nb {
 
-// Runtime switches of the record / weight-gradient experiments (NERF_B200_DBG_* environment variables: kernel variants without the
-// record copies, without the spare-warp sums, per-job finish times, per-warp wait cycles).  Compiled out of the product build;
-// `NERF_B200_EXPERIMENTS=1 python -c "import __graft_entry__ as g; g.build(force=True)"` builds them in.  The numbers under
-// profiles/r02_*_experiments* come from such a build.
-#ifdef NERF_B200_EXPERIMENTS
-constexpr bool kExp = true;
-#else
-constexpr bool kExp = false;
-#endif
-
 struct TilePlan {
   long long N; int S;
   int grid;            // CTAs of the forward launch (even: whole CTA pairs)

@@ -105,36 +105,6 @@ def test_empty_and_single_ray(G):
     assert rel_l2(r1["rgb_map"].cpu().numpy(), ref["rgb_map"]) < 2e-4
 
 
-def test_cta_pair_kernel_matches_single_cta_kernel():
-    """The default cta_group::2 pair kernel (fused_tc2.cuh) and the single-CTA kernel it superseded
-    (fused_tc.cuh, NERF_B200_PAIR=0) give the same results to fp32 accumulation-order noise.  Run in a subprocess because the mode is latched at first launch."""
-    import os, subprocess, sys
-    code = r'''
-import os, sys, numpy as np, torch
-sys.path.insert(0, os.getcwd()); sys.path.insert(0, os.path.join(os.getcwd(), "tests"))
-import gpu_common as G
-sb = G.synth.ray_batch("lego", 777, seed=5)
-nets = [G.make_net(G.synth.nerf_state(0)), G.make_net(G.synth.nerf_state(1))]
-with torch.no_grad():
-    r = G.nb.render(400, 400, sb["K"], rays=G.dev(sb["rays"]), ndc=False, near=2., far=6., use_viewdirs=True, network_fn=nets[0],
-                    network_fine=nets[1], network_query_fn=G.query_fn(), N_samples=64, N_importance=128, perturb=0.,
-                    white_bkgd=True, raw_noise_std=0.)
-np.save(sys.argv[1], torch.cat([r[0], r[1][:, None], r[2][:, None], r[3]["rgb0"]], -1).cpu().numpy())
-'''
-    import tempfile
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    outs = []
-    with tempfile.TemporaryDirectory() as tmp:
-        for mode in ("0", "1"):
-            path = os.path.join(tmp, f"o{mode}.npy")
-            env = dict(os.environ, NERF_B200_PAIR=mode)
-            subprocess.run([sys.executable, "-c", code, path], check=True, cwd=root, env=env, timeout=300)
-            outs.append(np.load(path))
-    assert rel_l2(outs[1][:, :3], outs[0][:, :3]) < 2e-5
-    assert rel_l2(outs[1][:, 4], outs[0][:, 4]) < 2e-5
-    assert rel_l2(outs[1][:, 5:8], outs[0][:, 5:8]) < 2e-5
-
-
 def test_graphed_render_matches_render(G):
     """GraphedRender replays exactly the kernels render() launches: bit-identical maps, also after a weight update."""
     sb = G.synth.ray_batch("lego", 513, seed=7)
